@@ -11,6 +11,7 @@ gathered/encoded into the peer ring (k_send) and deframed/scattered/cleared out 
     python bench.py [--gpus N] [--steps K] [--warmup W]
     torchrun ... bench.py --gpus N ...          (one rank per GPU, connections sharded, weak scaling)
     python bench.py --impl reference ...        (the reference's own CPU code on the host cores)
+    python bench.py --dump-outputs DIR ...      (also save what the last timed step delivered, as .npy)
 
 Prints ONE JSON line (see DESIGN.md "Measurement").
 """
@@ -25,6 +26,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the source tree, bytecode caches included
 
 MSG_BYTES = 4 * 1024 * 1024
 RING_KB = 16384
@@ -59,7 +61,14 @@ def parse():
     ap.add_argument("--unary-iters", type=int, default=2000)
     ap.add_argument("--service-workers", type=int, default=16)
     ap.add_argument("--stagger", type=int, default=0, help="1 = de-correlate the connections' ring positions first")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step delivered (rank 0) to "
+                    "DIR/<name>.npy, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 arm only")
+    return args
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -214,7 +223,7 @@ def reference_arm(args):
     threads = min(cores, conns)
     # one "step" = one message on every connection, like the B200 arm; W untimed + K timed steps
     # in ONE run of the multi-threaded harness (pairs are set up once, outside the timed region)
-    steps_done = max(1, min(args.steps, 200))
+    steps_done = args.steps
     t_total, _ = cpu_sample(eng, lens, conns, ring, threads, steps_done, warm=max(1, args.warmup))
     n_total = conns * steps_done
     gbs = n_total * args.msg_bytes / t_total / 1e9
@@ -418,6 +427,8 @@ def main():
     assert last.results(sh) == [total] * conns and br.results(sh) == [total] * conns
     # the LAST timed step's payload (the step before it carried the other one)
     assert torch.equal(srcs[(nstep[0] - 1) & 1], dst), "last timed step did not deliver its bytes"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dst, last.results(sh), br.results(sh))
     if world > 1:
         t = torch.tensor([t_dev_ms], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -529,6 +540,28 @@ def main():
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+DUMP_SAMPLES = 1 << 21
+DUMP_SEED = 20250101
+
+
+def dump_outputs(out_dir, dst, sent, received):
+    """--dump-outputs: what a caller of the timed path receives from its last step -- the bytes each send batch
+    consumed and each recv batch delivered per connection, and the delivered bytes themselves.  Those are 1 GiB at
+    the default size, so a fixed sample of positions (same seed, same positions on every run) is stored with its
+    indices: 24 MiB in all."""
+    import numpy as np
+    import torch
+    n = dst.numel()
+    idx = np.unique(np.random.default_rng(DUMP_SEED).integers(0, n, min(DUMP_SAMPLES, n)))
+    sample = dst[torch.from_numpy(idx).to(dst.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("send_bytes", np.asarray(sent, dtype=np.float64)),
+                    ("recv_bytes", np.asarray(received, dtype=np.float64)),
+                    ("delivered_sample_index", idx.astype(np.float64)),
+                    ("delivered_sample", sample.astype(np.float32))):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_nvlink_pass(pkg, L, dist, dev, stream, sh, rank, world, ring_kb, msg, conns=64, steps=4):

@@ -20,6 +20,7 @@ def test_reference_arm_prints_the_contract_line():
               "cpu_baseline", "e2e"):
         assert k in line, k
     assert line["value"] > 0 and line["gpu_launches"] == 0
+    assert line["steps"] == 2
     assert line["cpu_baseline"]["kind"] in ("reference", "port") and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0
 
